@@ -1,8 +1,8 @@
 #!/usr/bin/env python
-"""bench.py -- hot-path benchmark (contract in the task statement, tier section (4)).
+"""bench.py -- hot-path benchmark: prints one JSON result line.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4]
-                    [--rows R]
+                    [--rows R] [--dump-outputs DIR]
 
 A "step" is one pass of convert_from_rows over the whole synthetic workload.
   value      : rows/s with the JCUDF row buffer already resident in HBM (CUDA events, max over ranks)
@@ -491,6 +491,69 @@ def synth_c3_host(types, n, null_frac, seed):
     return cols
 
 
+def gather_ranges(torch, buf, starts, lens):
+    """buf[starts[0]:starts[0] + lens[0]] ++ buf[starts[1]:...] ++ ... (int64 device tensors), on the device."""
+    ends = torch.cumsum(lens, 0)
+    pos = torch.arange(int(ends[-1]), device=buf.device)
+    pos += torch.repeat_interleave(starts - (ends - lens), lens)
+    return buf[pos]
+
+
+def dump_c3(dirname, torch, types, nb, outs, direction):
+    """--dump-outputs: what the last timed step handed its caller, as DIR/<name>.npy (values exact in float64 / float32).
+    A step cycles over the resident pool, so slot k holds the output of every round i with i % pool == k.  A slot is a
+    whole batch of several GB: the same seeded sample of S rows of every slot is written.
+      rows                              [S]            the sampled row indices of a batch
+      from_rows: valid                  [pool, S, ncols]   validity bits
+                 fixed_words            [pool, S, W]       the fixed-width values as little-endian int32 words, column order
+                 string_starts, string_lengths [pool, S, nstr]  offsets[row] and offsets[row + 1] - offsets[row]
+                 string_chars           [chars]            the chars of the sampled strings, slot, column, row order
+      to_rows:   row_starts, row_lengths [pool, S]         offsets[row] and the row's length in bytes
+                 row_words              [words]            the sampled rows as little-endian int32 words, slot, row order"""
+    dev = outs[0]["cols"][0].mask.device if direction == "from_rows" else outs[0]["offs"].device
+    rows = np.sort(np.random.default_rng(0).choice(nb, min(nb, 1024 if direction == "from_rows" else 512), replace=False))
+    rows[0], rows[-1] = 0, nb - 1                          # the first and last row of a batch are always in the sample
+    idx = torch.from_numpy(rows).to(dev)
+    res = {"rows": rows.astype(np.float64)}
+    if direction == "from_rows":
+        valid, words, starts, lens, chars = [], [], [], [], []
+        for o in outs:
+            v, w, s_, l_ = [], [], [], []
+            for c in o["cols"]:
+                v.append((c.mask[idx // 32] >> (idx % 32).to(torch.int32)) & 1)
+                if c.dtype.type_id == STRING:
+                    offs = c.offsets.long()
+                    s, n = offs[idx], offs[idx + 1] - offs[idx]
+                    s_.append(s); l_.append(n)
+                    chars.append(gather_ranges(torch, c.data, s, n))
+                else:
+                    w.append(c.data.view(nb, SIZE[c.dtype.type_id])[idx].contiguous().view(torch.int32))
+            valid.append(torch.stack(v, 1))
+            words.append(torch.cat(w, 1))
+            starts.append(torch.stack(s_, 1))
+            lens.append(torch.stack(l_, 1))
+        res["valid"] = torch.stack(valid).cpu().numpy().astype(np.float32)
+        res["fixed_words"] = torch.stack(words).cpu().numpy().astype(np.float64)
+        res["string_starts"] = torch.stack(starts).cpu().numpy().astype(np.float64)
+        res["string_lengths"] = torch.stack(lens).cpu().numpy().astype(np.float64)
+        res["string_chars"] = torch.cat(chars).cpu().numpy().astype(np.float32)
+    else:
+        starts, lens, words = [], [], []
+        for o in outs:
+            offs = o["offs"].long()
+            s, n = offs[idx], offs[idx + 1] - offs[idx]
+            starts.append(s); lens.append(n)
+            words.append(gather_ranges(torch, o["data"], s, n).view(torch.int32))   # JCUDF rows are 8-byte multiples
+        res["row_starts"] = torch.stack(starts).cpu().numpy().astype(np.float64)
+        res["row_lengths"] = torch.stack(lens).cpu().numpy().astype(np.float64)
+        res["row_words"] = torch.cat(words).cpu().numpy().astype(np.float64)
+    total = sum(a.nbytes for a in res.values())
+    assert total <= 64 << 20, f"--dump-outputs: {total} bytes exceed 64 MB"
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in res.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def run_c3(args, wl, rank, world):
     import ctypes as C
 
@@ -722,6 +785,8 @@ def run_c3(args, wl, rank, world):
         torch.cuda.cudart().cudaProfilerStop()
     ms_gather = timed(True, args.steps) if do_gather else None    # conversion + all-gather, inside the step
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_c3(args.dump_outputs, torch, types, nb, outs, args.direction)
     ms_per_step = ms_gather if do_gather else ms_convert
     rows_step = rounds * nb                                       # rows one rank converts per step
     value = world * rows_step / (ms_per_step * 1e-3)
@@ -1370,7 +1435,14 @@ def main():
     ap.add_argument("--no-gather", action="store_true", help="multi-GPU: skip the all-gather (conversion-only scaling)")
     ap.add_argument("--gather", default="p2p", choices=["p2p", "nccl"],
                     help="multi-GPU all-gather transport: copy engines over NVLink peer memory (default) or ncclAllGather")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="c3: after the timed steps, write a fixed seeded sample of what the last step computed as DIR/<name>.npy "
+                         "(rank 0; same arguments give the same inputs, so two builds can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c3"):
+        ap.error("--dump-outputs is implemented for --workload c3 --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
