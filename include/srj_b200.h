@@ -267,7 +267,8 @@ SRJ_API int srj_partition_strings(const srj_column* in, const srj_column* out, i
  *                             SRJ_EINVAL on a malformed header.  The workspace keeps what srj_kudo_assemble needs.
  *   srj_kudo_assemble       : fills `out` (total_rows rows per column; null masks, where given, are produced for every
  *                             column -- partitions without validity contribute valid rows).
- * <= 256 columns, <= 65535 partitions.  LIST / STRUCT columns are not supported (SRJ_EUNSUPPORTED).
+ * <= 256 columns, <= 65535 partitions.  LIST / STRUCT columns are not supported here (SRJ_EUNSUPPORTED); nested tables
+ * are assembled by srj_kudo_assemble_nested below.
  */
 SRJ_API int64_t srj_kudo_workspace_bytes(int32_t num_columns, int32_t num_partitions);
 SRJ_API int srj_kudo_split_sizes(const srj_column* cols, int32_t num_columns, int64_t num_rows, const int32_t* d_splits,
@@ -280,6 +281,29 @@ SRJ_API int srj_kudo_assemble_sizes(const uint8_t* partitions, const int64_t* d_
                                     void* workspace, void* stream);
 SRJ_API int srj_kudo_assemble(const uint8_t* partitions, const int64_t* d_partition_offsets, int32_t num_partitions,
                               const srj_column* out, int32_t num_columns, int64_t total_rows, void* workspace, void* stream);
+
+/* Assemble of NESTED tables (LIST / STRUCT columns; a map is LIST<STRUCT<K, V>>).  The schema is flattened in pre-order
+ * (a LIST / STRUCT before its children), exactly as the reader's Schema gives it (getFlattenedTypeIds /
+ * getFlattenedNumChildren); the partitions may come from any Kudo writer, including the reference's host
+ * KudoSerializer (KudoTableHeaderCalc.java:77-195, SlicedBufferSerializer.java:72-247).
+ *   srj_kudo_nested_workspace_bytes : workspace of the two calls below (kept between them).
+ *   srj_kudo_assemble_nested_sizes  : per flattened column its assembled rows flat_rows[c] and, for STRING, chars
+ *                                     char_totals[c] (host arrays of num_flat; one stream synchronisation).
+ *                                     SRJ_EINVAL: the child counts do not describe the columns, a LIST does not have
+ *                                     exactly one child, or a partition is malformed (a section outside the partition's
+ *                                     bytes, offsets with off[0] < 0 or off[n] < off[0]).  SRJ_EOVERFLOW: a column's
+ *                                     rows or chars exceed INT32_MAX.
+ *   srj_kudo_assemble_nested        : fills the srj_column trees `out` (num_columns roots) of that schema: every column
+ *                                     flat_rows[c] rows, LIST / STRING offsets int32[rows + 1], STRING chars, LIST
+ *                                     children[0], STRUCT children; null masks, where given, are produced.
+ * <= 256 flattened columns, <= 65535 partitions.
+ */
+SRJ_API int64_t srj_kudo_nested_workspace_bytes(int32_t num_flat, int32_t num_partitions);
+SRJ_API int srj_kudo_assemble_nested_sizes(const uint8_t* partitions, const int64_t* d_partition_offsets, int32_t num_partitions,
+                                           const int32_t* flat_type_ids, const int32_t* flat_num_children, int32_t num_flat,
+                                           int64_t* flat_rows, int64_t* char_totals, void* workspace, void* stream);
+SRJ_API int srj_kudo_assemble_nested(const uint8_t* partitions, const int64_t* d_partition_offsets, int32_t num_partitions,
+                                     const srj_column* out, int32_t num_columns, void* workspace, void* stream);
 
 /* ---- Apache Spark UnsafeRow codec (SURVEY 8f rank 3) -----------------------------------------------------------
  * The row format Spark's own operators consume (org.apache.spark.sql.catalyst.expressions.UnsafeRow /

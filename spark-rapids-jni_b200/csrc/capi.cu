@@ -881,8 +881,9 @@ int srj_kudo_assemble_sizes(const uint8_t* partitions, const int64_t* d_partitio
   if ((num_partitions > 0 && !partitions) || !total_rows || !char_totals) { set_error("kudo_assemble_sizes: bad argument"); return SRJ_EINVAL; }
   rc = launch_kudo_assemble_sizes(partitions, d_partition_offsets, num_partitions, type_ids, num_columns, total_rows, char_totals, workspace,
                                   static_cast<cudaStream_t>(stream));
-  if (rc == SRJ_EINVAL) set_error("kudo_assemble_sizes: a partition does not start with a Kudo header of %d columns", num_columns);
+  if (rc == SRJ_EINVAL) set_error("kudo_assemble_sizes: a partition is not a well-formed Kudo partition of %d columns", num_columns);
   else if (rc == SRJ_EUNSUPPORTED) set_error("kudo_assemble_sizes: only fixed-width, decimal and STRING columns");
+  else if (rc == SRJ_EOVERFLOW) set_error("kudo_assemble_sizes: the assembled rows or chars of a column exceed INT32_MAX");
   else if (rc == SRJ_OK && *total_rows > INT32_MAX) { set_error("kudo_assemble_sizes: %lld rows exceed a column", static_cast<long long>(*total_rows)); return SRJ_EOVERFLOW; }
   return rc;
 }
@@ -897,6 +898,39 @@ int srj_kudo_assemble(const uint8_t* partitions, const int64_t* d_partition_offs
     if (out[c].size != total_rows) { set_error("kudo_assemble: column %d: expected %lld rows", c, static_cast<long long>(total_rows)); return SRJ_EINVAL; }
   rc = launch_kudo_assemble(partitions, d_partition_offsets, num_partitions, out, num_columns, total_rows, workspace, static_cast<cudaStream_t>(stream));
   if (rc == SRJ_EUNSUPPORTED) set_error("kudo_assemble: only fixed-width, decimal and STRING columns");
+  return rc;
+}
+
+int64_t srj_kudo_nested_workspace_bytes(int32_t num_flat, int32_t num_partitions)
+{
+  return kudo_workspace_bytes(std::max(num_flat, 0), std::max(num_partitions, 0));
+}
+
+int srj_kudo_assemble_nested_sizes(const uint8_t* partitions, const int64_t* d_partition_offsets, int32_t num_partitions, const int32_t* flat_type_ids,
+                                   const int32_t* flat_num_children, int32_t num_flat, int64_t* flat_rows, int64_t* char_totals, void* workspace,
+                                   void* stream)
+{
+  SRJ_API_RANGE();
+  int rc = kudo_check("kudo_assemble_nested_sizes", num_flat, num_partitions, flat_type_ids, d_partition_offsets, workspace);
+  if (rc != SRJ_OK) return rc;
+  if ((num_partitions > 0 && !partitions) || !flat_num_children || !flat_rows || !char_totals) { set_error("kudo_assemble_nested_sizes: bad argument"); return SRJ_EINVAL; }
+  rc = launch_kudo_assemble_nested_sizes(partitions, d_partition_offsets, num_partitions, flat_type_ids, flat_num_children, num_flat, flat_rows, char_totals,
+                                         workspace, static_cast<cudaStream_t>(stream));
+  if (rc == SRJ_EINVAL) set_error("kudo_assemble_nested_sizes: the flattened schema is not a forest of %d columns (a LIST has one child), or a partition is not a well-formed Kudo partition of it", num_flat);
+  else if (rc == SRJ_EUNSUPPORTED) set_error("kudo_assemble_nested_sizes: a type outside fixed-width, decimal, STRING, LIST and STRUCT");
+  else if (rc == SRJ_EOVERFLOW) set_error("kudo_assemble_nested_sizes: the assembled rows or chars of a column exceed INT32_MAX");
+  return rc;
+}
+
+int srj_kudo_assemble_nested(const uint8_t* partitions, const int64_t* d_partition_offsets, int32_t num_partitions, const srj_column* out,
+                             int32_t num_columns, void* workspace, void* stream)
+{
+  SRJ_API_RANGE();
+  int rc = kudo_check("kudo_assemble_nested", num_columns, num_partitions, out, d_partition_offsets, workspace);
+  if (rc != SRJ_OK) return rc;
+  rc = launch_kudo_assemble_nested(partitions, d_partition_offsets, num_partitions, out, num_columns, workspace, static_cast<cudaStream_t>(stream));
+  if (rc == SRJ_EINVAL) set_error("kudo_assemble_nested: malformed column tree (a LIST has one child and offsets, children are given)");
+  else if (rc == SRJ_EUNSUPPORTED) set_error("kudo_assemble_nested: more than 256 flattened columns, or a type outside the format");
   return rc;
 }
 

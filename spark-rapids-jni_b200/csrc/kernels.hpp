@@ -100,7 +100,7 @@ int launch_unsafe_from_rows(const srj_column* out, int32_t ncols, int64_t n, con
 int launch_unsafe_from_rows_strings(const srj_column* out, int32_t ncols, int64_t n, const uint8_t* rows, const int32_t* d_row_offsets,
                                     cudaStream_t stream);
 
-// ---- kudo.cu: the Kudo shuffle wire format for flat tables (split / assemble) ----
+// ---- kudo.cu: the Kudo shuffle wire format (split of flat tables / assemble of flat and nested tables) ----
 int64_t kudo_workspace_bytes(int32_t ncols, int32_t P);
 int launch_kudo_split_sizes(const srj_column* cols, int32_t ncols, const int32_t* d_splits, int32_t P, int64_t* d_part_offsets, int64_t* h_total,
                             void* workspace, cudaStream_t stream);
@@ -110,5 +110,10 @@ int launch_kudo_assemble_sizes(const uint8_t* buf, const int64_t* d_part_offsets
                                int64_t* h_char_totals, void* workspace, cudaStream_t stream);
 int launch_kudo_assemble(const uint8_t* buf, const int64_t* d_part_offsets, int32_t P, const srj_column* out, int32_t ncols, int64_t total_rows,
                          void* workspace, cudaStream_t stream);
+// nested (LIST / STRUCT) schemas, flattened in pre-order; the flat entry points above are these over a schema of leaves
+int launch_kudo_assemble_nested_sizes(const uint8_t* buf, const int64_t* d_part_offsets, int32_t P, const int32_t* type_ids, const int32_t* num_children,
+                                      int32_t F, int64_t* h_rows, int64_t* h_char_totals, void* workspace, cudaStream_t stream);
+int launch_kudo_assemble_nested(const uint8_t* buf, const int64_t* d_part_offsets, int32_t P, const srj_column* out, int32_t ncols, void* workspace,
+                                cudaStream_t stream);
 
 }  // namespace srj

@@ -11,11 +11,19 @@
 //               multiple of 4 (KudoSerializer.java:497-499)
 //   offsets   = per STRING column the n + 1 raw int32 offsets (not rebased), when n > 0; data = per column n * size bytes
 //               or the chars; both sections padded to 4
-// Flat tables only (fixed-width, decimals, STRING): the nested walk of the reference is not restated.
+// Split writes flat tables (fixed-width, decimals, STRING).  Assemble also reads nested tables (LIST / STRUCT columns,
+// KudoTableHeaderCalc.java:77-195, SlicedBufferSerializer.java:72-247, KudoTableMerger.java:96-295): the columns are
+// flattened in pre-order (a LIST / STRUCT before its children) and the column count and hasValidity bits index that
+// list; every flattened column has a slice (offset, rows): the header's at the root, the parent's below a STRUCT,
+// (off[0], off[n] - off[0]) of the list's raw offsets below a LIST.  Validity comes for STRUCT, LIST and leaf columns,
+// offsets for LIST and STRING columns, data for leaves, each in pre-order.  A flat table is a schema of leaves.
 //
-// Kernels: a thread per partition sizes it (and, for assemble, parses its header); one CTA per (column, partition)
-// moves that column's three buffers with the widest accesses the two addresses allow; validity bits of assembled
-// partitions reach the output words with atomicOr (a partition starts at an arbitrary row).
+// Kernels: split -- a thread per partition sizes it; one CTA per (column, partition) moves that column's buffers.
+// Assemble -- a thread per partition checks its header and walks the flattened schema once, recording per (column,
+// partition) the slice and where the column's buffers lie (every read is checked against the partition's bytes); one
+// CTA per column scans the partitions for row and char bases; one CTA per (column, partition) moves the buffers with
+// the widest accesses the two addresses allow.  Validity bits reach the output words with atomicOr (a slice starts at
+// an arbitrary row); LIST offsets are rebased onto the child's row base.
 #include <algorithm>
 #include <vector>
 
@@ -27,12 +35,16 @@ namespace srj {
 constexpr int kKudoMaxCols   = 256;
 constexpr uint32_t kKudoMagic = 0x4B554430u;
 
+enum : int32_t { KK_FIXED = 0, KK_STRING = 1, KK_LIST = 2, KK_STRUCT = 3 };
+
 struct KCol {
   uint8_t* data;        // fixed-width values or chars
   uint8_t* mask;        // validity bytes (bit r%8 of byte r/8), or NULL
-  int32_t* offsets;     // STRING
-  int32_t size;         // element bytes, 0 for STRING
-  int32_t sidx;         // index among the STRING columns, or -1
+  int32_t* offsets;     // STRING / LIST
+  int32_t size;         // element bytes, 0 for STRING / LIST / STRUCT
+  int32_t kind;         // KK_*
+  int32_t parent;       // flattened index of the parent column, -1 at the root
+  int32_t pad;
 };
 
 __host__ __device__ __forceinline__ int64_t pad4(int64_t x) { return (x + 3) & ~int64_t{3}; }
@@ -102,8 +114,9 @@ __global__ void __launch_bounds__(256) kudo_split_sizes_kernel(const KCol* __res
   if (n < 0 || pad4(hs + V) - hs + pad4(O) + pad4(D) > INT32_MAX) atomicExch(bad, 1);
 }
 
-// exclusive scan of P + 1 int64 in place by one CTA (P <= a few 10^4); element P receives the total
-__global__ void __launch_bounds__(1024) i64_scan_small_kernel(int64_t* v, int n)
+// exclusive scan of n values by one CTA of 1024 threads (n <= a few 10^4): put(i, sum of get(0 .. i - 1)) for i <= n
+template <class Get, class Put>
+__device__ void cta_exclusive_scan(int n, Get get, Put put)
 {
   __shared__ int64_t s_warp[32];
   __shared__ int64_t s_carry;
@@ -112,7 +125,7 @@ __global__ void __launch_bounds__(1024) i64_scan_small_kernel(int64_t* v, int n)
   const int lane = lane_id(), w = warp_id();
   for (int b = 0; b < n + 1; b += 1024) {
     const int i     = b + threadIdx.x;
-    const int64_t x = i < n ? v[i] : 0;
+    const int64_t x = i < n ? get(i) : 0;
     int64_t inc     = x;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -132,11 +145,17 @@ __global__ void __launch_bounds__(1024) i64_scan_small_kernel(int64_t* v, int n)
     }
     __syncthreads();
     const int64_t base = s_carry + (w > 0 ? s_warp[w - 1] : 0);
-    if (i <= n) v[i] = base + inc - x;
+    if (i <= n) put(i, base + inc - x);
     __syncthreads();
     if (threadIdx.x == 0) s_carry += s_warp[31];
     __syncthreads();
   }
+}
+
+// exclusive scan of P + 1 int64 in place by one CTA; element P receives the total
+__global__ void __launch_bounds__(1024) i64_scan_small_kernel(int64_t* v, int n)
+{
+  cta_exclusive_scan(n, [&](int i) { return v[i]; }, [&](int i, int64_t x) { v[i] = x; });
 }
 
 __global__ void __launch_bounds__(256) kudo_split_kernel(const KCol* __restrict__ cols, int ncols, const int32_t* __restrict__ splits,
@@ -196,95 +215,127 @@ struct KPartInfo {   // per partition, parsed from its header
   int32_t row_offset, rows, vlen, olen;
 };
 
+struct KRec {        // per (flattened column, partition)
+  int32_t off, rows;    // the column's slice in this partition
+  int32_t v, o, d;      // where its validity / offsets / data bytes start inside the three sections
+  int32_t has_v;        // validity bytes present
+  int64_t row_base;     // rows of the column in the partitions before this one
+  int64_t char_base;    // STRING: chars of the partition, then (scanned) chars before it
+};
+
 __device__ __forceinline__ uint32_t ld_be32(const uint8_t* p) { return (uint32_t{p[0]} << 24) | (uint32_t{p[1]} << 16) | (uint32_t{p[2]} << 8) | p[3]; }
 __device__ __forceinline__ int32_t ld_le32(const uint8_t* p) { return static_cast<int32_t>(uint32_t{p[0]} | (uint32_t{p[1]} << 8) | (uint32_t{p[2]} << 16) | (uint32_t{p[3]} << 24)); }
 
-// positions (from the start of the partition) of column c's buffers; *chars = bytes of its data buffer
-__device__ void kudo_locate(const uint8_t* part, const KPartInfo& pi, const int32_t* sizes /* element size per column, 0 = STRING */, int ncols, int c,
-                            bool* has_v, int64_t* v_at, int64_t* o_at, int64_t* d_at, int64_t* dbytes)
-{
-  const int hs = kudo_header_bytes(ncols);
-  const int n = pi.rows, s = pi.row_offset;
-  const int64_t vb = n > 0 ? (s + n - 1) / 8 - s / 8 + 1 : 0;
-  int64_t v = hs, o = hs + pi.vlen, d = hs + static_cast<int64_t>(pi.vlen) + pi.olen;
-  for (int k = 0; k <= c; ++k) {
-    const bool hv = (part[28 + k / 8] >> (k % 8)) & 1;
-    int64_t db;
-    const int64_t ob = (sizes[k] == 0 && n > 0) ? 4 * (static_cast<int64_t>(n) + 1) : 0;
-    if (sizes[k] == 0) db = ob ? static_cast<int64_t>(ld_le32(part + o + 4 * n)) - ld_le32(part + o) : 0;
-    else db = static_cast<int64_t>(n) * sizes[k];
-    if (k == c) {
-      *has_v = hv;
-      *v_at = v; *o_at = o; *d_at = d; *dbytes = db;
-      return;
-    }
-    if (hv) v += vb;
-    o += ob;
-    d += db;
-  }
-}
-
-// thread per partition: header -> KPartInfo, rows; *bad set on a malformed header
-__global__ void __launch_bounds__(256) kudo_parse_kernel(const uint8_t* __restrict__ buf, const int64_t* __restrict__ part_offsets, int P, int ncols,
-                                                        KPartInfo* __restrict__ info, int64_t* __restrict__ row_base /* [P + 1]: rows, scanned later */,
+// thread per partition: checks the header, walks the flattened schema in pre-order and fills rec[c * P + p].  The bytes
+// arrive over the network, so every section must lie inside [offs[p], offs[p + 1]) and every offsets pair read must
+// satisfy 0 <= off[0] <= off[n]; otherwise *bad is set and the partition contributes no rows.
+__global__ void __launch_bounds__(256) kudo_parse_kernel(const uint8_t* __restrict__ buf, const int64_t* __restrict__ part_offsets, int P, int F,
+                                                        const KCol* __restrict__ cols, KPartInfo* __restrict__ info, KRec* __restrict__ rec,
                                                         int32_t* __restrict__ bad)
 {
   const int p = blockIdx.x * 256 + threadIdx.x;
   if (p >= P) return;
-  const uint8_t* h = buf + part_offsets[p];
-  KPartInfo pi{static_cast<int32_t>(ld_be32(h + 4)), static_cast<int32_t>(ld_be32(h + 8)), static_cast<int32_t>(ld_be32(h + 12)),
-               static_cast<int32_t>(ld_be32(h + 16))};
-  if (ld_be32(h) != kKudoMagic || static_cast<int>(ld_be32(h + 24)) != ncols || pi.rows < 0 || pi.row_offset < 0) {
+  const int64_t plen = part_offsets[p + 1] - part_offsets[p];
+  const int hs       = kudo_header_bytes(F);
+  const uint8_t* h   = buf + part_offsets[p];
+  KPartInfo pi{0, 0, 0, 0};
+  bool ok = plen >= hs;
+  int64_t dlen = 0;
+  if (ok) {
+    pi = KPartInfo{static_cast<int32_t>(ld_be32(h + 4)), static_cast<int32_t>(ld_be32(h + 8)), static_cast<int32_t>(ld_be32(h + 12)),
+                   static_cast<int32_t>(ld_be32(h + 16))};
+    const int32_t total = static_cast<int32_t>(ld_be32(h + 20));
+    dlen = static_cast<int64_t>(total) - pi.vlen - pi.olen;
+    ok = ld_be32(h) == kKudoMagic && static_cast<int>(ld_be32(h + 24)) == F && pi.rows >= 0 && pi.row_offset >= 0 && pi.vlen >= 0 &&
+         pi.olen >= 0 && dlen >= 0 && hs + static_cast<int64_t>(total) <= plen;
+  }
+  const uint8_t* os = h + hs + (ok ? pi.vlen : 0);
+  int64_t v = 0, o = 0, d = 0;
+  for (int c = 0; ok && c < F; ++c) {
+    const KCol col = cols[c];
+    KRec r{};
+    if (col.parent < 0) {
+      r.off = pi.row_offset;
+      r.rows = pi.rows;
+    } else {
+      const KRec& from = rec[static_cast<int64_t>(cols[col.parent].kind == KK_STRUCT ? col.parent : c) * P + p];   // below a LIST: set by the list
+      r.off = from.off;
+      r.rows = from.rows;
+    }
+    const int32_t s = r.off, n = r.rows;
+    r.has_v = n > 0 && ((h[28 + c / 8] >> (c % 8)) & 1);
+    r.v = static_cast<int32_t>(v);
+    r.o = static_cast<int32_t>(o);
+    r.d = static_cast<int32_t>(d);
+    if (r.has_v) v += (static_cast<int64_t>(s) + n - 1) / 8 - s / 8 + 1;
+    if (col.kind == KK_STRING || col.kind == KK_LIST) {
+      int32_t a = 0, b = 0;
+      if (n > 0) {
+        const int64_t ob = 4 * (static_cast<int64_t>(n) + 1);
+        if (o + ob > pi.olen) { ok = false; break; }
+        a = ld_le32(os + o);
+        b = ld_le32(os + o + 4 * static_cast<int64_t>(n));
+        if (a < 0 || b < a) { ok = false; break; }
+        o += ob;
+      }
+      if (col.kind == KK_LIST) {
+        KRec& child = rec[static_cast<int64_t>(c + 1) * P + p];   // pre-order: a LIST's only child follows it
+        child.off   = a;
+        child.rows  = b - a;
+      } else {
+        r.char_base = b - a;
+        d += b - a;
+      }
+    } else if (col.kind == KK_FIXED) {
+      d += static_cast<int64_t>(n) * col.size;
+    }
+    if (v > pi.vlen || d > dlen) { ok = false; break; }
+    rec[static_cast<int64_t>(c) * P + p] = r;
+  }
+  if (!ok) {
     atomicExch(bad, 1);
     pi.rows = 0;
+    for (int c = 0; c < F; ++c) rec[static_cast<int64_t>(c) * P + p] = KRec{};
   }
-  info[p]     = pi;
-  row_base[p] = pi.rows;
+  info[p] = pi;
 }
 
-// chars of every (STRING column, partition): thread per STRING column walks the partitions (exclusive prefix in place)
-__global__ void __launch_bounds__(64) kudo_chars_kernel(const uint8_t* __restrict__ buf, const int64_t* __restrict__ part_offsets, int P, int ncols,
-                                                       const int32_t* __restrict__ sizes, const int32_t* __restrict__ scols, int nstr,
-                                                       const KPartInfo* __restrict__ info, int64_t* __restrict__ chars_base /* [nstr][P + 1] */)
+// CTA per flattened column: row_base / char_base of every partition (exclusive scans); totals[2c] = rows, [2c + 1] = chars
+__global__ void __launch_bounds__(1024) kudo_scan_kernel(KRec* __restrict__ rec, int P, int64_t* __restrict__ totals)
 {
-  const int k = blockIdx.x * 64 + threadIdx.x;
-  if (k >= nstr) return;
-  int64_t run = 0;
-  for (int p = 0; p < P; ++p) {
-    bool hv;
-    int64_t v, o, d, db;
-    kudo_locate(buf + part_offsets[p], info[p], sizes, ncols, scols[k], &hv, &v, &o, &d, &db);
-    chars_base[static_cast<int64_t>(k) * (P + 1) + p] = run;
-    run += db;
-  }
-  chars_base[static_cast<int64_t>(k) * (P + 1) + P] = run;
+  const int c = blockIdx.x;
+  KRec* r     = rec + static_cast<int64_t>(c) * P;
+  cta_exclusive_scan(P, [&](int i) { return static_cast<int64_t>(r[i].rows); },
+                     [&](int i, int64_t x) { if (i < P) r[i].row_base = x; else totals[2 * c] = x; });
+  cta_exclusive_scan(P, [&](int i) { return r[i].char_base; },
+                     [&](int i, int64_t x) { if (i < P) r[i].char_base = x; else totals[2 * c + 1] = x; });
 }
 
-__global__ void __launch_bounds__(256) kudo_assemble_kernel(const uint8_t* __restrict__ buf, const int64_t* __restrict__ part_offsets, int P, int ncols,
-                                                           const int32_t* __restrict__ sizes, const KCol* __restrict__ out, const KPartInfo* __restrict__ info,
-                                                           const int64_t* __restrict__ row_base, const int64_t* __restrict__ chars_base)
+// 5 CTAs per SM (<= 51 registers, no spills): the copy is bound by loads in flight, and the unconstrained build's 62
+// registers would leave 4
+__global__ void __launch_bounds__(256, 5) kudo_assemble_kernel(const uint8_t* __restrict__ buf, const int64_t* __restrict__ part_offsets, int P, int F,
+                                                           const KCol* __restrict__ out, const KPartInfo* __restrict__ info, const KRec* __restrict__ rec)
 {
   const int c = blockIdx.x, p = blockIdx.y;
-  const KPartInfo pi = info[p];
-  const int n = pi.rows;
+  const KRec r = rec[static_cast<int64_t>(c) * P + p];
+  const int n  = r.rows;
   if (n == 0) return;
-  const uint8_t* part = buf + part_offsets[p];
-  __shared__ int64_t s_at[4];
-  __shared__ bool s_hv;
-  if (threadIdx.x == 0) kudo_locate(part, pi, sizes, ncols, c, &s_hv, &s_at[0], &s_at[1], &s_at[2], &s_at[3]);
-  __syncthreads();
-  const KCol col   = out[c];
-  const int64_t rb = row_base[p];
-  // ---- validity: output bits [rb, rb + n) <- input bits [row_offset % 8, ... ) of the partition's bytes, or ones ----
+  const KPartInfo pi  = info[p];
+  const uint8_t* vs   = buf + part_offsets[p] + kudo_header_bytes(F);
+  const uint8_t* os   = vs + pi.vlen;
+  const uint8_t* ds   = os + pi.olen;
+  const KCol col      = out[c];
+  const int64_t rb    = r.row_base;
+  // ---- validity: output bits [rb, rb + n) <- input bits [off % 8, ... ) of the slice's bytes, or ones ----
   if (col.mask) {
-    const uint8_t* vb   = part + s_at[0];
-    const int shift     = pi.row_offset & 7;
+    const uint8_t* vb   = vs + r.v;
+    const int shift     = r.off & 7;
     uint32_t* om        = reinterpret_cast<uint32_t*>(col.mask);
     const int64_t w0    = rb >> 5, w1 = (rb + n - 1) >> 5;
     for (int64_t w = w0 + threadIdx.x; w <= w1; w += 256) {
       const int64_t r_lo = tmax<int64_t>(rb, w << 5), r_hi = tmin<int64_t>(rb + n, (w + 1) << 5);   // rows of this word
       uint32_t bits = 0;
-      if (s_hv) {
+      if (r.has_v) {
         const int64_t i0 = r_lo - rb + shift;   // first input bit
         uint64_t acc     = 0;
         const int64_t nbytes = ((i0 & 7) + (r_hi - r_lo) + 7) >> 3;   // <= 5
@@ -299,16 +350,15 @@ __global__ void __launch_bounds__(256) kudo_assemble_kernel(const uint8_t* __res
       if (bits) atomicOr(om + w, bits);
     }
   }
-  // ---- offsets + chars, or fixed-width data ----
-  if (sizes[c] == 0) {
-    const uint8_t* ob = part + s_at[1];
-    int sidx          = col.sidx;
-    const int64_t cb  = chars_base[static_cast<int64_t>(sidx) * (P + 1) + p];
-    const int32_t o0  = ld_le32(ob);
-    for (int i = threadIdx.x; i <= n; i += 256) col.offsets[rb + i] = static_cast<int32_t>(cb + (ld_le32(ob + 4 * static_cast<int64_t>(i)) - o0));
-    cta_copy_bytes(col.data + cb, part + s_at[2], s_at[3]);
-  } else {
-    cta_copy_bytes(col.data + rb * sizes[c], part + s_at[2], s_at[3]);
+  // ---- offsets (rebased onto the child's rows or the chars before the partition) + chars, or fixed-width data ----
+  if (col.kind == KK_STRING || col.kind == KK_LIST) {
+    const uint8_t* ob  = os + r.o;
+    const int64_t base = col.kind == KK_LIST ? rec[static_cast<int64_t>(c + 1) * P + p].row_base : r.char_base;
+    const int32_t o0   = ld_le32(ob);
+    for (int i = threadIdx.x; i <= n; i += 256) col.offsets[rb + i] = static_cast<int32_t>(base + (ld_le32(ob + 4 * static_cast<int64_t>(i)) - o0));
+    if (col.kind == KK_STRING) cta_copy_bytes(col.data + base, ds + r.d, ld_le32(ob + 4 * static_cast<int64_t>(n)) - o0);
+  } else if (col.kind == KK_FIXED) {
+    cta_copy_bytes(col.data + rb * col.size, ds + r.d, static_cast<int64_t>(n) * col.size);
   }
 }
 
@@ -328,62 +378,46 @@ static int kudo_elem_size(int32_t t)
   }
 }
 
-// workspace: [KCol x 256 | sizes int32 x 256 | scols int32 x 256 | bad flag (64 B) | KPartInfo x P | row_base int64 x (P + 1) | chars_base int64 x nstr x (P + 1)]
+// workspace: [KCol x 256 | bad flag (64 B) | totals int64 x 2 x 256 | KPartInfo x P | KRec x F x P]
 struct KudoWs {
   KCol* cols;
-  int32_t* sizes;
-  int32_t* scols;
   int32_t* bad;
+  int64_t* totals;
   KPartInfo* info;
-  int64_t* row_base;
-  int64_t* chars_base;
+  KRec* rec;
 };
 static KudoWs kudo_ws(void* workspace, int P)
 {
   uint8_t* w = static_cast<uint8_t*>(workspace);
   KudoWs k;
-  k.cols  = reinterpret_cast<KCol*>(w);
+  k.cols = reinterpret_cast<KCol*>(w);
   w += kKudoMaxCols * sizeof(KCol);
-  k.sizes = reinterpret_cast<int32_t*>(w);
-  w += kKudoMaxCols * 4;
-  k.scols = reinterpret_cast<int32_t*>(w);
-  w += kKudoMaxCols * 4;
   k.bad = reinterpret_cast<int32_t*>(w);
   w += 64;
+  k.totals = reinterpret_cast<int64_t*>(w);
+  w += 2 * kKudoMaxCols * 8;
   k.info = reinterpret_cast<KPartInfo*>(w);
   w += (static_cast<size_t>(P) * sizeof(KPartInfo) + 63) & ~size_t{63};
-  k.row_base = reinterpret_cast<int64_t*>(w);
-  w += ((static_cast<size_t>(P) + 1) * 8 + 63) & ~size_t{63};
-  k.chars_base = reinterpret_cast<int64_t*>(w);
+  k.rec = reinterpret_cast<KRec*>(w);
   return k;
 }
 int64_t kudo_workspace_bytes(int32_t ncols, int32_t P)
 {
-  return static_cast<int64_t>(kKudoMaxCols) * (sizeof(KCol) + 8) + 64 + static_cast<int64_t>(P) * sizeof(KPartInfo) + 64 +
-         (static_cast<int64_t>(P) + 1) * 8 + 64 + static_cast<int64_t>(std::max(ncols, 1)) * (static_cast<int64_t>(P) + 1) * 8 + 256;
+  return static_cast<int64_t>(kKudoMaxCols) * (sizeof(KCol) + 16) + 64 + static_cast<int64_t>(P) * sizeof(KPartInfo) + 64 +
+         static_cast<int64_t>(std::max(ncols, 1)) * P * sizeof(KRec) + 256;
 }
 
-static int kudo_upload(const srj_column* cols, int32_t ncols, const KudoWs& ws, int* nstr_out, cudaStream_t stream)
+static int kudo_upload(const srj_column* cols, int32_t ncols, const KudoWs& ws, cudaStream_t stream)
 {
   if (ncols <= 0 || ncols > kKudoMaxCols) return SRJ_EUNSUPPORTED;
   KCol h[kKudoMaxCols];
-  int32_t sizes[kKudoMaxCols], scols[kKudoMaxCols];
-  int nstr = 0;
   for (int c = 0; c < ncols; ++c) {
     const int sz = kudo_elem_size(cols[c].type_id);
     if (sz < 0) return SRJ_EUNSUPPORTED;
-    h[c].data    = static_cast<uint8_t*>(cols[c].data);
-    h[c].mask    = reinterpret_cast<uint8_t*>(cols[c].null_mask);
-    h[c].offsets = cols[c].offsets;
-    h[c].size    = sz;
-    h[c].sidx    = sz == 0 ? nstr : -1;
-    sizes[c]     = sz;
-    if (sz == 0) scols[nstr++] = c;
+    h[c] = KCol{static_cast<uint8_t*>(cols[c].data), reinterpret_cast<uint8_t*>(cols[c].null_mask), cols[c].offsets, sz,
+                sz == 0 ? KK_STRING : KK_FIXED, -1, 0};
   }
   SRJ_CUDA_TRY(cudaMemcpyAsync(ws.cols, h, sizeof(KCol) * ncols, cudaMemcpyHostToDevice, stream));
-  SRJ_CUDA_TRY(cudaMemcpyAsync(ws.sizes, sizes, 4 * ncols, cudaMemcpyHostToDevice, stream));
-  if (nstr) SRJ_CUDA_TRY(cudaMemcpyAsync(ws.scols, scols, 4 * nstr, cudaMemcpyHostToDevice, stream));
-  *nstr_out = nstr;
   return SRJ_OK;
 }
 
@@ -391,8 +425,7 @@ int launch_kudo_split_sizes(const srj_column* cols, int32_t ncols, const int32_t
                             void* workspace, cudaStream_t stream)
 {
   const KudoWs ws = kudo_ws(workspace, P);
-  int nstr = 0;
-  const int rc = kudo_upload(cols, ncols, ws, &nstr, stream);
+  const int rc = kudo_upload(cols, ncols, ws, stream);
   if (rc != SRJ_OK) return rc;
   SRJ_CUDA_TRY(cudaMemsetAsync(ws.bad, 0, 4, stream));
   kudo_split_sizes_kernel<<<(P + 255) / 256, 256, 0, stream>>>(ws.cols, ncols, d_splits, P, d_part_offsets, ws.bad);
@@ -409,60 +442,140 @@ int launch_kudo_split(const srj_column* cols, int32_t ncols, const int32_t* d_sp
                       void* workspace, cudaStream_t stream)
 {
   const KudoWs ws = kudo_ws(workspace, P);
-  int nstr = 0;
-  const int rc = kudo_upload(cols, ncols, ws, &nstr, stream);
+  const int rc = kudo_upload(cols, ncols, ws, stream);
   if (rc != SRJ_OK) return rc;
   kudo_split_kernel<<<dim3(ncols, P), 256, 0, stream>>>(ws.cols, ncols, d_splits, d_part_offsets, out);
   SRJ_CUDA_TRY(cudaGetLastError());
   return SRJ_OK;
 }
 
+// the flattened schema -> kind / size / parent of every column; SRJ_EINVAL when the child counts do not describe a
+// forest of `F` columns or a LIST has other than one child, SRJ_EUNSUPPORTED for a type outside the format
+static int kudo_schema(const int32_t* type_ids, const int32_t* num_children, int F, KCol* h)
+{
+  if (F <= 0) return SRJ_EINVAL;
+  if (F > kKudoMaxCols) return SRJ_EUNSUPPORTED;
+  int stack[kKudoMaxCols], left[kKudoMaxCols], depth = 0;
+  for (int c = 0; c < F; ++c) {
+    while (depth > 0 && left[depth - 1] == 0) --depth;
+    h[c] = KCol{nullptr, nullptr, nullptr, 0, KK_FIXED, depth > 0 ? stack[depth - 1] : -1, 0};
+    if (depth > 0) --left[depth - 1];
+    const int32_t t = type_ids[c], k = num_children[c];
+    if (t == SRJ_LIST || t == SRJ_STRUCT) {
+      if (k < 0 || (t == SRJ_LIST && k != 1)) return SRJ_EINVAL;
+      h[c].kind   = t == SRJ_LIST ? KK_LIST : KK_STRUCT;
+      stack[depth] = c;
+      left[depth++] = k;
+    } else {
+      const int sz = kudo_elem_size(t);
+      if (sz < 0) return SRJ_EUNSUPPORTED;
+      if (k != 0) return SRJ_EINVAL;
+      h[c].size = sz;
+      h[c].kind = sz == 0 ? KK_STRING : KK_FIXED;
+    }
+  }
+  while (depth > 0 && left[depth - 1] == 0) --depth;
+  return depth == 0 ? SRJ_OK : SRJ_EINVAL;
+}
+
+int launch_kudo_assemble_nested_sizes(const uint8_t* buf, const int64_t* d_part_offsets, int32_t P, const int32_t* type_ids, const int32_t* num_children,
+                                      int32_t F, int64_t* h_rows, int64_t* h_char_totals, void* workspace, cudaStream_t stream)
+{
+  const KudoWs ws = kudo_ws(workspace, P);
+  KCol h[kKudoMaxCols];
+  const int rc = kudo_schema(type_ids, num_children, F, h);
+  if (rc != SRJ_OK) return rc;
+  SRJ_CUDA_TRY(cudaMemcpyAsync(ws.cols, h, sizeof(KCol) * F, cudaMemcpyHostToDevice, stream));
+  SRJ_CUDA_TRY(cudaMemsetAsync(ws.bad, 0, 4, stream));
+  if (P > 0) kudo_parse_kernel<<<(P + 255) / 256, 256, 0, stream>>>(buf, d_part_offsets, P, F, ws.cols, ws.info, ws.rec, ws.bad);
+  kudo_scan_kernel<<<F, 1024, 0, stream>>>(ws.rec, P, ws.totals);
+  SRJ_CUDA_TRY(cudaGetLastError());
+  int32_t bad = 0;
+  std::vector<int64_t> totals(2 * static_cast<size_t>(F));
+  SRJ_CUDA_TRY(cudaMemcpyAsync(&bad, ws.bad, 4, cudaMemcpyDeviceToHost, stream));
+  SRJ_CUDA_TRY(cudaMemcpyAsync(totals.data(), ws.totals, 16 * static_cast<size_t>(F), cudaMemcpyDeviceToHost, stream));
+  SRJ_CUDA_TRY(cudaStreamSynchronize(stream));
+  if (bad) return SRJ_EINVAL;
+  bool over = false;
+  for (int c = 0; c < F; ++c) {
+    h_rows[c]        = totals[2 * c];
+    h_char_totals[c] = totals[2 * c + 1];
+    over |= h_rows[c] > INT32_MAX || h_char_totals[c] > INT32_MAX;   // int32 offsets / size_type rows
+  }
+  return over ? SRJ_EOVERFLOW : SRJ_OK;
+}
+
+// the srj_column trees in pre-order
+static int kudo_flatten(const srj_column* cols, int32_t n, std::vector<const srj_column*>& flat)
+{
+  for (int32_t i = 0; i < n; ++i) {
+    if (static_cast<int>(flat.size()) >= kKudoMaxCols) return SRJ_EUNSUPPORTED;
+    flat.push_back(&cols[i]);
+    const int32_t t = cols[i].type_id;
+    if (t == SRJ_LIST || t == SRJ_STRUCT) {
+      if (cols[i].num_children > 0 && !cols[i].children) return SRJ_EINVAL;
+      const int rc = kudo_flatten(cols[i].children, cols[i].num_children, flat);
+      if (rc != SRJ_OK) return rc;
+    }
+  }
+  return SRJ_OK;
+}
+
+int launch_kudo_assemble_nested(const uint8_t* buf, const int64_t* d_part_offsets, int32_t P, const srj_column* out, int32_t ncols, void* workspace,
+                                cudaStream_t stream)
+{
+  const KudoWs ws = kudo_ws(workspace, P);
+  std::vector<const srj_column*> flat;
+  int rc = kudo_flatten(out, ncols, flat);
+  if (rc != SRJ_OK) return rc;
+  const int F = static_cast<int>(flat.size());
+  int32_t ids[kKudoMaxCols], nch[kKudoMaxCols];
+  for (int c = 0; c < F; ++c) {
+    ids[c] = flat[c]->type_id;
+    nch[c] = (ids[c] == SRJ_LIST || ids[c] == SRJ_STRUCT) ? flat[c]->num_children : 0;
+  }
+  KCol h[kKudoMaxCols];
+  rc = kudo_schema(ids, nch, F, h);
+  if (rc != SRJ_OK) return rc;
+  for (int c = 0; c < F; ++c) {
+    const srj_column& o = *flat[c];
+    h[c].data    = static_cast<uint8_t*>(o.data);
+    h[c].mask    = reinterpret_cast<uint8_t*>(o.null_mask);
+    h[c].offsets = o.offsets;
+    if (o.null_mask && o.size > 0) SRJ_CUDA_TRY(cudaMemsetAsync(o.null_mask, 0, static_cast<size_t>((o.size + 31) / 32) * 4, stream));
+    if (h[c].kind == KK_STRING || h[c].kind == KK_LIST) {
+      if (!o.offsets) return SRJ_EINVAL;
+      if (o.size == 0) SRJ_CUDA_TRY(cudaMemsetAsync(o.offsets, 0, 4, stream));
+    }
+  }
+  SRJ_CUDA_TRY(cudaMemcpyAsync(ws.cols, h, sizeof(KCol) * F, cudaMemcpyHostToDevice, stream));
+  if (P > 0) kudo_assemble_kernel<<<dim3(F, P), 256, 0, stream>>>(buf, d_part_offsets, P, F, ws.cols, ws.info, ws.rec);
+  SRJ_CUDA_TRY(cudaGetLastError());
+  return SRJ_OK;
+}
+
+// flat tables: a schema of leaves
 int launch_kudo_assemble_sizes(const uint8_t* buf, const int64_t* d_part_offsets, int32_t P, const int32_t* type_ids, int32_t ncols, int64_t* h_rows,
                                int64_t* h_char_totals, void* workspace, cudaStream_t stream)
 {
-  const KudoWs ws = kudo_ws(workspace, P);
   if (ncols <= 0 || ncols > kKudoMaxCols) return SRJ_EUNSUPPORTED;
-  int32_t sizes[kKudoMaxCols], scols[kKudoMaxCols];
-  int nstr = 0;
-  for (int c = 0; c < ncols; ++c) {
-    sizes[c] = kudo_elem_size(type_ids[c]);
-    if (sizes[c] < 0) return SRJ_EUNSUPPORTED;
-    if (sizes[c] == 0) scols[nstr++] = c;
-    h_char_totals[c] = 0;
-  }
-  SRJ_CUDA_TRY(cudaMemcpyAsync(ws.sizes, sizes, 4 * ncols, cudaMemcpyHostToDevice, stream));
-  if (nstr) SRJ_CUDA_TRY(cudaMemcpyAsync(ws.scols, scols, 4 * nstr, cudaMemcpyHostToDevice, stream));
-  SRJ_CUDA_TRY(cudaMemsetAsync(ws.bad, 0, 4, stream));
-  kudo_parse_kernel<<<(P + 255) / 256, 256, 0, stream>>>(buf, d_part_offsets, P, ncols, ws.info, ws.row_base, ws.bad);
-  i64_scan_small_kernel<<<1, 1024, 0, stream>>>(ws.row_base, P);
-  if (nstr) kudo_chars_kernel<<<(nstr + 63) / 64, 64, 0, stream>>>(buf, d_part_offsets, P, ncols, ws.sizes, ws.scols, nstr, ws.info, ws.chars_base);
-  SRJ_CUDA_TRY(cudaGetLastError());
-  int32_t bad = 0;
-  std::vector<int64_t> totals(static_cast<size_t>(std::max(nstr, 1)));
-  SRJ_CUDA_TRY(cudaMemcpyAsync(&bad, ws.bad, 4, cudaMemcpyDeviceToHost, stream));
-  SRJ_CUDA_TRY(cudaMemcpyAsync(h_rows, ws.row_base + P, 8, cudaMemcpyDeviceToHost, stream));
-  for (int k = 0; k < nstr; ++k)
-    SRJ_CUDA_TRY(cudaMemcpyAsync(&totals[k], ws.chars_base + static_cast<int64_t>(k) * (P + 1) + P, 8, cudaMemcpyDeviceToHost, stream));
-  SRJ_CUDA_TRY(cudaStreamSynchronize(stream));
-  if (bad) return SRJ_EINVAL;
-  for (int k = 0; k < nstr; ++k) h_char_totals[scols[k]] = totals[k];
-  return SRJ_OK;
+  for (int c = 0; c < ncols; ++c)
+    if (kudo_elem_size(type_ids[c]) < 0) return SRJ_EUNSUPPORTED;
+  const std::vector<int32_t> leaves(ncols, 0);
+  std::vector<int64_t> rows(ncols);
+  const int rc = launch_kudo_assemble_nested_sizes(buf, d_part_offsets, P, type_ids, leaves.data(), ncols, rows.data(), h_char_totals, workspace, stream);
+  if (rc == SRJ_OK || rc == SRJ_EOVERFLOW) *h_rows = rows[0];
+  return rc;
 }
 
 int launch_kudo_assemble(const uint8_t* buf, const int64_t* d_part_offsets, int32_t P, const srj_column* out, int32_t ncols, int64_t total_rows,
                          void* workspace, cudaStream_t stream)
 {
-  const KudoWs ws = kudo_ws(workspace, P);
-  int nstr = 0;
-  const int rc = kudo_upload(out, ncols, ws, &nstr, stream);   // (sizes / scols are rewritten with the same values)
-  if (rc != SRJ_OK) return rc;
-  for (int c = 0; c < ncols; ++c) {
-    if (out[c].null_mask && total_rows > 0) SRJ_CUDA_TRY(cudaMemsetAsync(out[c].null_mask, 0, static_cast<size_t>((total_rows + 31) / 32) * 4, stream));
-    if (out[c].type_id == SRJ_STRING && total_rows == 0) SRJ_CUDA_TRY(cudaMemsetAsync(out[c].offsets, 0, 4, stream));
-  }
-  if (P > 0) kudo_assemble_kernel<<<dim3(ncols, P), 256, 0, stream>>>(buf, d_part_offsets, P, ncols, ws.sizes, ws.cols, ws.info, ws.row_base, ws.chars_base);
-  SRJ_CUDA_TRY(cudaGetLastError());
-  return SRJ_OK;
+  if (ncols <= 0 || ncols > kKudoMaxCols) return SRJ_EUNSUPPORTED;
+  for (int c = 0; c < ncols; ++c)
+    if (kudo_elem_size(out[c].type_id) < 0) return SRJ_EUNSUPPORTED;
+  (void)total_rows;   // = out[c].size, checked by the caller
+  return launch_kudo_assemble_nested(buf, d_part_offsets, P, out, ncols, workspace, stream);
 }
 
 }  // namespace srj

@@ -25,7 +25,7 @@ import torch
 from . import _native as N
 from ._native import CudfColumnSizeOverflowException, CudfException, CudaException  # noqa: F401
 
-__all__ = ["DType", "ColumnVector", "ColumnView", "Table", "RowConversion", "Hash", "CudfException",
+__all__ = ["DType", "Schema", "ColumnVector", "ColumnView", "Table", "RowConversion", "Hash", "CudfException",
            "CudfColumnSizeOverflowException", "Plan"]
 
 
@@ -61,6 +61,71 @@ class DType:
 
     def __repr__(self):
         return f"DType({self.type_id}, scale={self.scale})"
+
+
+class Schema:
+    """ai.rapids.cudf.Schema: the column types of a table as a tree (LIST / STRUCT columns have children), and its
+    pre-order flattening -- the form the Kudo reader takes (KudoGpuSerializer.assembleFromDeviceRaw).
+
+        b = Schema.builder()
+        b.column(DType(DType.INT64), "key")
+        lst = b.addColumn(DType(DType.LIST), "xs"); lst.column(DType(DType.INT32), "x")
+        schema = b.build()
+    """
+
+    class Builder:
+        def __init__(self, dtype: Optional["DType"] = None, name: Optional[str] = None):
+            self.dtype, self.name = dtype, name
+            self.children: List["Schema.Builder"] = []
+
+        def addColumn(self, dtype, name: str) -> "Schema.Builder":
+            """Add a column; for LIST and STRUCT the returned builder takes its children, otherwise this builder."""
+            child = Schema.Builder(_as_dtype(dtype), name)
+            self.children.append(child)
+            return child if child.dtype.type_id in (DType.LIST, DType.STRUCT) else self
+
+        def column(self, dtype, name: str) -> "Schema.Builder":
+            self.addColumn(dtype, name)
+            return self
+
+        def build(self) -> "Schema":
+            return Schema(self)
+
+    def __init__(self, root: "Schema.Builder"):
+        self._root = root
+
+    @staticmethod
+    def builder() -> "Schema.Builder":
+        return Schema.Builder()
+
+    def _flat(self) -> List["Schema.Builder"]:
+        out: List[Schema.Builder] = []
+
+        def go(b):
+            out.append(b)
+            for k in b.children:
+                go(k)
+        for k in self._root.children:
+            go(k)
+        return out
+
+    def getColumnNames(self) -> List[str]:
+        return [k.name for k in self._root.children]
+
+    def getNumChildren(self) -> int:
+        return len(self._root.children)
+
+    def getFlattenedNumColumns(self) -> int:
+        return len(self._flat())
+
+    def getFlattenedTypeIds(self) -> List[int]:
+        return [b.dtype.type_id for b in self._flat()]
+
+    def getFlattenedNumChildren(self) -> List[int]:
+        return [len(b.children) for b in self._flat()]
+
+    def getFlattenedTypeScales(self) -> List[int]:
+        return [b.dtype.scale for b in self._flat()]
 
 
 def _as_dtype(d) -> DType:

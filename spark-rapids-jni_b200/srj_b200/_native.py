@@ -86,6 +86,10 @@ SYMBOLS = {
     "srj_kudo_assemble_sizes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int64),
                                           C.POINTER(C.c_int64), C.c_void_p, C.c_void_p]),
     "srj_kudo_assemble": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.POINTER(SrjColumn), C.c_int32, C.c_int64, C.c_void_p, C.c_void_p]),
+    "srj_kudo_nested_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32]),
+    "srj_kudo_assemble_nested_sizes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int32,
+                                                 C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_void_p, C.c_void_p]),
+    "srj_kudo_assemble_nested": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.POINTER(SrjColumn), C.c_int32, C.c_void_p, C.c_void_p]),
     "srj_shard_rebase_offsets": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
                                            C.c_int32, C.c_int32, C.c_void_p]),
     "srj_convert_from_rows_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.POINTER(SrjColumn),
